@@ -1,6 +1,6 @@
 """Benchmark of the hot path: seconds-of-audio per second separated (n_fft=2048, hop=1024).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = the whole inference hot path (STFT -> sliding windows -> CascadedNet -> mask -> 2x inverse STFT,
@@ -20,6 +20,9 @@ one mask gather to rank 0 before the overlap-add).  Prints ONE JSON line (rank 0
   mgpu_check (N > 1) sharded vs single-GPU stems on a 31 s track, with and without --tta; the run fails above 1e-5
 --impl reference runs only that CPU arm (the reference itself is Python over librosa and cannot travel to the
 GPU box; oracle/ is its restatement, validated against the unmodified reference in tests/).
+--dump-outputs DIR writes the stems the last timed step returned (rank 0) as DIR/instruments.npy and DIR/vocals.npy,
+float32 (2, n).  Inputs and checkpoint are seeded, so two builds can be compared output for output; stems larger than
+the 60 MB budget are sampled at the same seeded, sorted sample positions in every run.
 """
 import argparse
 import json
@@ -48,6 +51,7 @@ CONV_FLOP_PER_WINDOW = 135.714e9   # SURVEY.md 8(d)
 # was fused); the un-fused minimum of SURVEY 8(d) is 1.142 GB/window.
 CONV_DRAM_BYTES_PER_WINDOW = 0.903e9
 GOLDEN = os.path.join(ROOT, 'tests', 'golden', 'ref_10s_default.npz')
+DUMP_BYTES = 60_000_000   # --dump-outputs: all files together, .npy headers included
 
 
 def measured_peaks():
@@ -136,6 +140,19 @@ def cpu_reference_arm(steps, warmup, sample_seconds=18.0):
     return sample_seconds / dt, dt, cores, sample_seconds
 
 
+def dump_outputs(outdir, stems):
+    """Writes every (channels, samples) CUDA tensor of ``stems`` as outdir/<name>.npy (float32).  A stem whose share of
+    DUMP_BYTES cannot hold it whole keeps a seeded, sorted sample of its sample positions, all channels."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in stems.items():
+        rows, n = t.shape
+        cols = min(n, (DUMP_BYTES // len(stems) - 128) // (4 * rows))   # 128: the .npy header
+        if cols < n:
+            pos = np.sort(np.random.default_rng(0).choice(n, cols, replace=False))
+            t = t[:, torch.from_numpy(pos).to(t.device)]
+        np.save(os.path.join(outdir, name + '.npy'), t.cpu().numpy())
+
+
 def workload_text(seconds, n_windows, batch):
     return ('%d s 44.1 kHz stereo synthetic track (240 s per GPU, BASELINE configs[2]), %d windows of cropsize 256, '
             'window batch %d; seeded synthetic checkpoint (lib/synth.py)' % (int(seconds), n_windows, batch))
@@ -145,7 +162,7 @@ def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     warm = max(1, min(args.warmup, 1))
     val, dt, cores, secs = cpu_reference_arm(steps, warm)
     seconds = args.seconds_per_gpu * max(1, args.gpus)
@@ -316,16 +333,21 @@ def run_gpu(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps, per_step=None):
+    def timed(fn, steps, per_step=None, last=None):
         """K steps bracketed by barrier + synchronize, CUDA events on the launching stream, max over ranks.  per_step
-        (a list) additionally receives every step's own duration (events between steps cost nothing measurable)."""
+        (a list) additionally receives every step's own duration (events between steps cost nothing measurable);
+        last (a list) receives what the last step returned."""
         barrier()
         evs = [torch.cuda.Event(enable_timing=True) for _ in range(steps + 1)]
         evs[0].record()
+        out = None
         for i in range(steps):
-            fn()
+            out = None   # every step starts with the previous step's output released, as when it is not kept
+            out = fn()
             evs[i + 1].record()
         barrier()
+        if last is not None:
+            last.append(out)
         ms = evs[0].elapsed_time(evs[steps])
         each = [evs[i].elapsed_time(evs[i + 1]) for i in range(steps)]
         if world > 1:
@@ -348,10 +370,14 @@ def run_gpu(args):
     sampler.start()
     launches0 = ctx.launch_count()
     per_step = []
-    ms = timed(step_device, args.steps, per_step)
+    last = []
+    ms = timed(step_device, args.steps, per_step, last)
     launches = ctx.launch_count() - launches0
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(('instruments', 'vocals'), last[0])))
+    del last
     ms_step = ms / args.steps
     value = seconds / (ms_step * 1e-3)
     ms_median = sorted(per_step)[len(per_step) // 2]
@@ -533,8 +559,14 @@ def main():
     ap.add_argument('--no-strong', action='store_true', help='skip the 40-minute strong-scaling sub-record')
     ap.add_argument('--seconds-per-gpu', type=float, default=SECONDS_PER_GPU,
                     help='track length per GPU (default 240 s = BASELINE configs[2]; shorter only for profiling)')
+    ap.add_argument('--dump-outputs', type=str, default='', metavar='DIR',
+                    help='write the stems of the last timed step to DIR/instruments.npy and DIR/vocals.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
     if args.impl == 'reference':
+        if args.dump_outputs:
+            ap.error('--dump-outputs writes the stems of the GPU path; --impl reference times a CPU sample')
         run_reference(args)
     else:
         run_gpu(args)

@@ -122,6 +122,43 @@ def run_case(name, seconds, n_fft, hop, nout, nout_lstm, cropsize, batchsize, fs
     print('wrote', path, os.path.getsize(path) // 1024, 'KiB')
 
 
+def merge_artifacts_masks():
+    """Six seeded (2, 33, 400) masks: low-level noise with one to three long above-threshold runs."""
+    rng = np.random.default_rng(0)
+    masks = []
+    for trial in range(6):
+        m = rng.uniform(0.0, 0.04, size=(2, 33, 400)).astype(np.float32)
+        for s, e in ((0, 90), (150, 260), (275, 400))[:1 + trial % 3]:
+            m[:, :, s:e] = rng.uniform(0.06, 1.0, size=(2, 33, e - s))
+        masks.append(m)
+    return masks
+
+
+def run_functions(name):
+    """Reference outputs of two single functions: ``CascadedNet.predict_mask`` (lib/nets.py:124-131) on the first
+    256-frame window of the 10 s input with the default net, and ``spec_utils.merge_artifacts`` (lib/spec_utils.py:60-93)
+    on ``merge_artifacts_masks()``.  Stored sampled over bins, with float64 checksums of the full arrays."""
+    ref_inference, ref_nets, ref_spec_utils, ref_dataset = librosa_shim.import_reference()
+    from lib import synth
+    sd = synth.to_torch_state_dict(synth.make_state_dict())
+    model = ref_nets.CascadedNet(2048, 1024, 32, 128)
+    model.load_state_dict(sd)
+    model.eval()
+    X = ref_spec_utils.wave_to_spectrogram(synth.sine_mix(10.0), 1024, 2048)
+    pad_l, pad_r, roi = ref_dataset.make_padding(X.shape[2], 256, model.offset)
+    Xp = np.pad(X, ((0, 0), (0, 0), (pad_l, pad_r)))
+    Xp /= np.abs(X).max()
+    with torch.no_grad():
+        pm = model.predict_mask(torch.from_numpy(np.abs(Xp[None, :, :, roi:roi + 256]))).numpy()
+    merged = [ref_spec_utils.merge_artifacts(m.copy()) for m in merge_artifacts_masks()]
+    out = dict(predict_mask_sub=pm[:, :, 4::8, :], predict_mask_sum=checksum(pm),
+               merge_artifacts_sub=np.stack([r[:, ::8, :] for r in merged]),
+               merge_artifacts_sum=np.stack([checksum(r) for r in merged]))
+    path = os.path.join(GOLDEN_DIR, name + '.npz')
+    np.savez_compressed(path, **out)
+    print('wrote', path, os.path.getsize(path) // 1024, 'KiB')
+
+
 class _Wrap(torch.nn.Module):
     def __init__(self, net, fn):
         super().__init__()
@@ -138,6 +175,7 @@ def main():
     run_case('ref_10s_default', 10.0, 2048, 1024, 32, 128, 256, 4, 8, 1, True, True)
     # a small configuration exercising the n_fft / cropsize / nout flags
     run_case('ref_3s_small', 3.0, 512, 256, 16, 32, 192, 2, 2, 1, False, False)
+    run_functions('ref_functions')
 
 
 if __name__ == '__main__':

@@ -44,6 +44,12 @@ def golden_small():
     return np.load(os.path.join(GOLDEN, 'ref_3s_small.npz'))
 
 
+@pytest.fixture(scope='session')
+def golden_functions():
+    import numpy as np
+    return np.load(os.path.join(GOLDEN, 'ref_functions.npz'))
+
+
 def checksum(a):
     import numpy as np
     a = np.asarray(a)

@@ -3,10 +3,12 @@ in lib/_native.py covers exactly that set.  No compute calls (there is no GPU in
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 
-from conftest import ROOT
+from conftest import PKG, ROOT
 
 
 def _declared():
@@ -33,12 +35,12 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_create_fails_loudly_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip('GPU present')
-    from lib import _native
-    with pytest.raises(_native.NativeError):
-        _native.Context(0, 2048, 1024, 32, 128, 256, 1)
+    """Run in a child process that sees no CUDA device, so that it checks the same thing on a GPU machine."""
+    code = ('import pytest\nfrom lib import _native\nwith pytest.raises(_native.NativeError):\n'
+            '    _native.Context(0, 2048, 1024, 32, 128, 256, 1)\n')
+    r = subprocess.run([sys.executable, '-c', code], cwd=PKG, env=dict(os.environ, CUDA_VISIBLE_DEVICES=''),
+                       capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
 
 
 def test_library_missing_is_an_error(monkeypatch, tmp_path):
