@@ -169,14 +169,31 @@ VR_API int vr_debug_conv(vr_ctx* ctx, const float* x, int32_t N, int32_t Cin, in
 VR_API int vr_debug_decoder(vr_ctx* ctx, const float* low, int32_t N, int32_t Cl, int32_t h, int32_t w, const float* skip,
                      int32_t Cs, const float* wgt, const float* bias, int32_t Cout, int32_t act, int32_t fused, float* y,
                      void* stream);
-/* Process-wide debug knobs of the tensor-core kernels: key 0 = 1 sets the UMMA matrix-base-offset field in the
- * row-streaming kernel's shifted descriptors (wrong on B200, kept for tests/diag_rows.py), key 1 = 1 disables that kernel, key 2 = 64 makes it use 64-channel (SW128) chunks instead of 32 (set before vr_create), key 3 = 1 enables the experimental flat-halo kernel (before vr_create), key 5 = 1 fuses the decoder upsample into
- * the row-streaming kernel (before vr_create).                  */
+/* Process-wide debug knobs of the tensor-core kernels (keys 0..7): key 0 = 1 records the row-streaming kernel's
+ * timeline for vr_debug_trace (builds with -DVR_TRACE), key 1 = 1 disables that kernel, key 2 = 1 makes vr_debug_conv use the row kernel's
+ * 64-output-channel tile, key 4 = k sets the number of interpolation slots of the fused upsample, key 5 = 1 (default)
+ * fuses the decoder upsample into the row-streaming kernel and lets vr_create choose the fused dec1 layouts (0: staged
+ * layout everywhere; set before vr_create), key 6 = 1 (default) skips 8-channel input groups whose weights are all
+ * zero.                                                                                                        */
 VR_API int vr_debug_set(int32_t key, int32_t value);
-/* Internal activation of the last forward as NCHW float32; dims receives [N,C,H,W].                       */
 /* timeline of CTA 0 of the last row-kernel launch made with vr_debug_set(0, 1): 3 roles x 2048 events x 3 clock64 stamps
  * (MMA issuer / TMA producer / interpolation warp 0), copied to HOST memory; returns the number of values or -1 */
 VR_API int64_t vr_debug_trace(uint64_t* host_out, int64_t capacity);
+/* Internal tensor of the last forward, copied to the DEVICE buffer out (capacity floats); dims receives 4 sizes.
+ * Activations (split-bf16 buffers, returned as hi + lo in float32 NCHW, every channel of the buffer incl. padding;
+ * dims = [N, C, H, W]):
+ *   "x", "aux1", "aux2"        slots of the stage input buffer, all max_bin rows ([0, bins/2) low band, rest high band)
+ *   "o1", "o2"                 stage-1 / stage-2 low-band BaseNet outputs before the 1x1 bridges
+ *   "f3"                       stage-3 output
+ *   "<k>.<buf>"                buffer of BaseNet k (0 stg1_low, 1 stg1_high, 2 stg2_low, 3 stg2_high, 4 stg3_full):
+ *                              cat1 cat2 cat3 cat4 (decoder concat inputs), t2 t3 t4 t5 (encoder conv1 outputs),
+ *                              e5, pool (ASPP frequency mean), f1, acat, ao, d4, d3, d2, and lstm_up (only for nets that
+ *                              keep the up-sampled LSTM channel in a buffer of its own; an error otherwise)
+ * LSTM branch fp32 planes of BaseNet k, copied raw (dims = the layout padded with 1s):
+ *   "<k>.lstm_l0"  [N, bins, T, 1]      1x1 input convolution, pre-activation sums
+ *   "<k>.lstm_xp"  [N, T, 8*hid, 1]     gate pre-activations, forward then reverse direction
+ *   "<k>.lstm_hs"  [N, T, 2*hid, 1]     hidden states, forward then reverse direction
+ *   "<k>.lstm_y"   [bins, N, T, 1]      dense + BatchNorm1d + ReLU output                                      */
 VR_API int vr_debug_read(vr_ctx* ctx, const char* what, float* out, int64_t capacity, int64_t* dims, void* stream);
 
 #ifdef __cplusplus

@@ -1055,17 +1055,39 @@ bool Engine::debug_read(const char* what, float* out, int64_t cap, int64_t* dims
   else if (w == "aux1") { v = in3_.view(N, 0, max_bin, pos_aux1_, nout / 4); C = nout / 4; }
   else if (w == "aux2") { v = in3_.view(N, 0, max_bin, pos_aux2_, nout / 2); C = nout / 2; }
   else if (w == "x") { v = in3_.view(N, 0, max_bin, pos_x_, 2); C = 2; }
+  else if (w == "o1") { v = o1_.all(N); C = o1_.C; }
+  else if (w == "o2") { v = o2_.all(N); C = o2_.C; }
   else {
     // "<net index>.<buffer>" e.g. "4.e5", "0.d2"
     int ni = w.size() > 2 && w[1] == '.' ? w[0] - '0' : -1;
     if (ni < 0 || ni > 4) { err = "debug_read: unknown tensor " + w; return false; }
     BaseNetPlan& P = nets_[ni];
     const std::string b = w.substr(2);
+    // the LSTM branch's fp32 planes, copied raw; dims are their LstmPlan layout padded with 1s
+    const LstmPlan& Q = P.lstm;
+    const float* plane = nullptr;
+    int64_t pd[4] = {0, 0, 0, 1};
+    if (b == "lstm_l0") { plane = Q.l0; pd[0] = N; pd[1] = Q.bins; pd[2] = Q.T; }
+    else if (b == "lstm_xp") { plane = Q.xp; pd[0] = N; pd[1] = Q.T; pd[2] = 8 * Q.hid; }
+    else if (b == "lstm_hs") { plane = Q.hs; pd[0] = N; pd[1] = Q.T; pd[2] = 2 * Q.hid; }
+    else if (b == "lstm_y") { plane = Q.y; pd[0] = Q.bins; pd[1] = N; pd[2] = Q.T; }
+    if (plane) {
+      const int64_t count = pd[0] * pd[1] * pd[2];
+      for (int i = 0; i < 4; ++i) dims[i] = pd[i];
+      if (count > cap) { err = "debug_read: output buffer too small"; return false; }
+      return ck(cudaMemcpyAsync(out, plane, sizeof(float) * (size_t)count, cudaMemcpyDeviceToDevice, s), "debug_read");
+    }
     const Buffer* buf = nullptr;
     if (b == "cat1") buf = &P.cat1; else if (b == "cat2") buf = &P.cat2; else if (b == "cat3") buf = &P.cat3;
     else if (b == "cat4") buf = &P.cat4; else if (b == "e5") buf = &P.e5; else if (b == "acat") buf = &P.acat;
     else if (b == "ao") buf = &P.ao; else if (b == "d4") buf = &P.d4; else if (b == "d3") buf = &P.d3;
     else if (b == "d2") buf = &P.d2; else if (b == "t2") buf = &P.t2; else if (b == "f1") buf = &P.f1;
+    else if (b == "t3") buf = &P.t3; else if (b == "t4") buf = &P.t4; else if (b == "t5") buf = &P.t5;
+    else if (b == "pool") buf = &P.pool;
+    else if (b == "lstm_up") {
+      if (!P.lstm_own) { err = "debug_read: " + P.prefix + " keeps its up-sampled LSTM channel in cat1, not lstm_up"; return false; }
+      buf = &P.lstm_up;
+    }
     else { err = "debug_read: unknown buffer " + b; return false; }
     v = buf->all(N); C = buf->C;
   }
