@@ -124,6 +124,25 @@ VR_API int vr_separate_wave(vr_ctx* ctx, const float* wave, int64_t L, int32_t t
 VR_API int vr_separate_wave_host(vr_ctx* ctx, const float* wave_host, int64_t L, int32_t tta, float* inst_host,
                           float* voc_host, void* stream);
 
+/* Several tracks per call (not a reference surface: the reference separates one file per run).  A track is cut into
+ * cropsize windows as in vr_separate; here the windows of ALL tracks share the forward batches of max_batch windows, so
+ * short tracks and the last partial batch of each track do not each pay for a nearly empty forward.  Windows are
+ * independent inside the net, and each track keeps its own normaliser and padding, so every mask equals the one
+ * vr_separate gives for that track alone.  Every argument is checked before anything is launched; an error names the
+ * offending track.
+ *
+ * vr_separate_many: Separator.separate / separate_tta (tta as in vr_separate) over n_tracks >= 1 tracks.  specs[i] is
+ * a complex64 [2][bins][T[i]] spectrogram (T[i] >= 1), masks[i] receives the float32 [2][bins][T[i]] mask.  specs, T and
+ * masks are HOST arrays of n_tracks entries; the pointers in specs and masks are DEVICE pointers.                   */
+VR_API int vr_separate_many(vr_ctx* ctx, int32_t n_tracks, const void* const* specs, const int64_t* T, int32_t tta,
+                            float* const* masks, void* stream);
+/* vr_separate_wave over n_tracks >= 1 tracks: waves[i] float32 [2][L[i]] (L[i] >= 0) -> inst[i], voc[i]
+ * [2][hop*(T_i-1)], T_i = 1 + L[i]/hop.  waves, L, inst and voc are HOST arrays of n_tracks entries holding DEVICE
+ * pointers.  The STFT, the normalisers and the masked inverse STFT of all tracks are one launch each; the
+ * workspaces grow with the total frame count of the call.                                                         */
+VR_API int vr_separate_waves(vr_ctx* ctx, int32_t n_tracks, const float* const* waves, const int64_t* L, int32_t tta,
+                             float* const* inst, float* const* voc, void* stream);
+
 /* The sample-rate conversion inside librosa.load(path, sr=args.sr, res_type='kaiser_fast') (inference.py:136-138,
  * pseudo.py:47-50) = resampy.resample(y, orig_sr, sr, filter='kaiser_fast'): x [channels][n_in] -> y [channels][n_out],
  * n_out = (int64)(n_in * sample_ratio), sample_ratio = sr / orig_sr.  win / delta: DEVICE float64 arrays of nwin entries -

@@ -191,6 +191,36 @@ int vr_separate_wave_host(vr_ctx* ctx, const float* wave_host, int64_t L, int32_
   return done(ctx, ctx->eng->separate_wave_host(wave_host, L, tta, inst_host, voc_host, (cudaStream_t)stream));
 }
 
+int vr_separate_many(vr_ctx* ctx, int32_t n_tracks, const void* const* specs, const int64_t* T, int32_t tta,
+                     float* const* masks, void* stream) {
+  CHECK_CTX(ctx);
+  // everything is checked before anything is launched
+  if (n_tracks < 1) return fail(ctx, "vr_separate_many: n_tracks must be >= 1");
+  if (!specs || !T || !masks) return fail(ctx, "vr_separate_many: specs, T and masks must not be NULL");
+  for (int32_t i = 0; i < n_tracks; ++i) {
+    const std::string at = "vr_separate_many: track " + std::to_string(i) + ": ";
+    if (!specs[i]) return fail(ctx, at + "specs[i] is NULL");
+    if (!masks[i]) return fail(ctx, at + "masks[i] is NULL");
+    if (T[i] < 1) return fail(ctx, at + "T[i] must be >= 1");
+  }
+  return done(ctx, ctx->eng->separate_many((const float2* const*)specs, T, n_tracks, tta, masks, (cudaStream_t)stream));
+}
+
+int vr_separate_waves(vr_ctx* ctx, int32_t n_tracks, const float* const* waves, const int64_t* L, int32_t tta,
+                      float* const* inst, float* const* voc, void* stream) {
+  CHECK_CTX(ctx);
+  if (n_tracks < 1) return fail(ctx, "vr_separate_waves: n_tracks must be >= 1");
+  if (!waves || !L || !inst || !voc) return fail(ctx, "vr_separate_waves: waves, L, inst and voc must not be NULL");
+  for (int32_t i = 0; i < n_tracks; ++i) {
+    const std::string at = "vr_separate_waves: track " + std::to_string(i) + ": ";
+    if (!waves[i]) return fail(ctx, at + "waves[i] is NULL");
+    if (!inst[i]) return fail(ctx, at + "inst[i] is NULL");
+    if (!voc[i]) return fail(ctx, at + "voc[i] is NULL");
+    if (L[i] < 0) return fail(ctx, at + "L[i] must be >= 0");
+  }
+  return done(ctx, ctx->eng->separate_waves(waves, L, n_tracks, tta, inst, voc, (cudaStream_t)stream));
+}
+
 int vr_resample(vr_ctx* ctx, const float* x, int32_t channels, int64_t n_in, float* y, int64_t n_out, double sample_ratio,
                 const double* win, const double* delta, int32_t nwin, int32_t table_per_crossing, void* stream) {
   // ctx may be NULL (audio is usually loaded before a model context exists): the call then runs on the calling

@@ -12,22 +12,14 @@
 namespace vr {
 
 // ------------------------------------------------------------------------------------------------
-__global__ void pack_mag_from_spec_kernel(const float2* __restrict__ spec, int bins, int64_t T, int max_bin, int W,
-                                          int roi, int pad_l, int first_window, const float* __restrict__ norm,
-                                          ActView dst) {
-  int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  int64_t total = (int64_t)dst.N * max_bin * W;
-  if (idx >= total) return;
-  int tw = (int)(idx % W);
-  int64_t r = idx / W;
-  int bin = (int)(r % max_bin);
-  int n = (int)(r / max_bin);
-  int64_t t = (int64_t)(first_window + n) * roi + tw - pad_l;
+// Frame tw of window `window` (|X|/norm, spectrogram padded by pad_l zeros) -> pixel (n, bin, tw) of dst.
+__device__ __forceinline__ void pack_mag_pixel(const float2* __restrict__ spec, int bins, int64_t T, int roi, int pad_l,
+                                               int window, float nv, ActView dst, int n, int bin, int tw) {
+  int64_t t = (int64_t)window * roi + tw - pad_l;
   // A silent track has max|X| = 0 (the reference then divides 0/0 and writes NaN stems for that one file).  Here a
   // NaN would outlive the call: stage-1/2 layers read the aux channel slots of the shared input buffer through zero
   // weights, and 0 * NaN = NaN inside the MMA would poison every later track on this context.  So a zero / non-finite
   // normaliser packs zeros, and non-finite magnitudes (NaN / Inf samples) are packed as zeros as well.
-  const float nv = *norm;
   const float inv = (nv > 0.f && nv <= 3.0e38f) ? 1.0f / nv : 0.f;
   float m0 = 0.f, m1 = 0.f;
   if (t >= 0 && t < T) {
@@ -44,6 +36,41 @@ __global__ void pack_mag_from_spec_kernel(const float2* __restrict__ spec, int b
   split_bf16(m1, h1, l1);
   *reinterpret_cast<__nv_bfloat162*>(dst.hi + off) = __halves2bfloat162(h0, h1);
   *reinterpret_cast<__nv_bfloat162*>(dst.lo + off) = __halves2bfloat162(l0, l1);
+}
+
+__global__ void pack_mag_from_spec_kernel(const float2* __restrict__ spec, int bins, int64_t T, int max_bin, int W,
+                                          int roi, int pad_l, int first_window, const float* __restrict__ norm,
+                                          ActView dst) {
+  int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int64_t total = (int64_t)dst.N * max_bin * W;
+  if (idx >= total) return;
+  int tw = (int)(idx % W);
+  int64_t r = idx / W;
+  int bin = (int)(r % max_bin);
+  int n = (int)(r / max_bin);
+  pack_mag_pixel(spec, bins, T, roi, pad_l, first_window + n, *norm, dst, n, bin, tw);
+}
+
+// Batch slot n packs window wins[n] of its own track with its track's normaliser.
+__global__ void pack_mag_many_kernel(const WinDesc* __restrict__ wins, int bins, int max_bin, int W, int roi,
+                                     const float* __restrict__ norms, ActView dst) {
+  int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int64_t total = (int64_t)dst.N * max_bin * W;
+  if (idx >= total) return;
+  int tw = (int)(idx % W);
+  int64_t r = idx / W;
+  int bin = (int)(r % max_bin);
+  int n = (int)(r / max_bin);
+  const WinDesc& d = wins[n];
+  pack_mag_pixel(d.spec, bins, d.T, roi, d.pad_l, d.window, norms[d.norm], dst, n, bin, tw);
+}
+
+cudaError_t launch_pack_mag_many(const WinDesc* wins, int bins, int max_bin, int W, int roi, const float* norms,
+                                 ActView dst, cudaStream_t stream) {
+  int64_t total = (int64_t)dst.N * max_bin * W;
+  if (total == 0) return cudaSuccess;
+  pack_mag_many_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(wins, bins, max_bin, W, roi, norms, dst);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_pack_mag_from_spec(const float2* spec, int bins, int64_t T, int max_bin, int W, int roi,
@@ -262,6 +289,45 @@ cudaError_t launch_broadcast_rows(ActView in, ActView out, cudaStream_t stream) 
 
 // ------------------------------------------------------------------------------------------------
 // Final 1x1 conv (nout -> 2, no BN) + sigmoid, only for the frames that survive the offset crop.
+// Kept frame tr of image n, row bin of f3 -> d0 (channel 0) and d0 + stride_c (channel 1); the Nyquist row is also
+// stored one row (stride_bin) further down.
+template <int NOUT>
+__device__ __forceinline__ void mask_out_pixel(const ActView& f3, const float* __restrict__ w, int offset, int n,
+                                               int bin, int tr, float* d0, int64_t stride_c, int64_t stride_bin,
+                                               int accumulate) {
+  int64_t o = (int64_t)n * f3.sn + (int64_t)bin * f3.sh + (int64_t)(tr + offset) * f3.sw;
+  float a0 = 0.f, a1 = 0.f;
+#pragma unroll
+  for (int c = 0; c < NOUT; c += 8) {
+    float x[8];
+    load8(f3.hi + o + c, f3.lo + o + c, x);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      a0 = fmaf(x[i], __ldg(w + c + i), a0);
+      a1 = fmaf(x[i], __ldg(w + NOUT + c + i), a1);
+    }
+  }
+  float m0 = 1.f / (1.f + expf(-a0));
+  float m1 = 1.f / (1.f + expf(-a1));
+  float* d1 = d0 + stride_c;
+  const bool last = bin == f3.H - 1;   // F.pad(..., mode='replicate') of the Nyquist row (lib/nets.py:111-115)
+  if (accumulate) {
+    *d0 = (*d0 + m0) * 0.5f;
+    *d1 = (*d1 + m1) * 0.5f;
+    if (last) {
+      d0[stride_bin] = (d0[stride_bin] + m0) * 0.5f;
+      d1[stride_bin] = (d1[stride_bin] + m1) * 0.5f;
+    }
+  } else {
+    *d0 = m0;
+    *d1 = m1;
+    if (last) {
+      d0[stride_bin] = m0;
+      d1[stride_bin] = m1;
+    }
+  }
+}
+
 template <int NOUT>
 __global__ void mask_out_kernel(MaskOutParams p) {
   const int roi = p.f3.W - 2 * p.offset;
@@ -274,38 +340,42 @@ __global__ void mask_out_kernel(MaskOutParams p) {
   int n = (int)(r / p.f3.H);
   int64_t t = p.t_base0 + (int64_t)n * p.roi_t + tr;
   if (t < 0 || t >= p.t_limit) return;
-  int64_t o = (int64_t)n * p.f3.sn + (int64_t)bin * p.f3.sh + (int64_t)(tr + p.offset) * p.f3.sw;
-  float a0 = 0.f, a1 = 0.f;
-#pragma unroll
-  for (int c = 0; c < NOUT; c += 8) {
-    float x[8];
-    load8(p.f3.hi + o + c, p.f3.lo + o + c, x);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      a0 = fmaf(x[i], __ldg(p.w + c + i), a0);
-      a1 = fmaf(x[i], __ldg(p.w + NOUT + c + i), a1);
-    }
-  }
-  float m0 = 1.f / (1.f + expf(-a0));
-  float m1 = 1.f / (1.f + expf(-a1));
   float* d0 = p.out + (int64_t)n * p.stride_n + (int64_t)bin * p.stride_bin + p.t_base0 + tr;
-  float* d1 = d0 + p.stride_c;
-  const bool last = bin == p.f3.H - 1;   // F.pad(..., mode='replicate') of the Nyquist row (lib/nets.py:111-115)
-  if (p.accumulate) {
-    *d0 = (*d0 + m0) * 0.5f;
-    *d1 = (*d1 + m1) * 0.5f;
-    if (last) {
-      d0[p.stride_bin] = (d0[p.stride_bin] + m0) * 0.5f;
-      d1[p.stride_bin] = (d1[p.stride_bin] + m1) * 0.5f;
-    }
-  } else {
-    *d0 = m0;
-    *d1 = m1;
-    if (last) {
-      d0[p.stride_bin] = m0;
-      d1[p.stride_bin] = m1;
-    }
+  mask_out_pixel<NOUT>(p.f3, p.w, p.offset, n, bin, tr, d0, p.stride_c, p.stride_bin, p.accumulate);
+}
+
+// Batch slot n writes into the mask of its own track: wins[n].mask [2][bins][T], frame t_base + tr.
+template <int NOUT>
+__global__ void mask_out_many_kernel(ActView f3, const float* __restrict__ w, int offset,
+                                     const WinDesc* __restrict__ wins) {
+  const int roi = f3.W - 2 * offset;
+  int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int64_t total = (int64_t)f3.N * f3.H * roi;
+  if (idx >= total) return;
+  int tr = (int)(idx % roi);
+  int64_t r = idx / roi;
+  int bin = (int)(r % f3.H);
+  int n = (int)(r / f3.H);
+  const WinDesc& d = wins[n];
+  const int64_t t = d.t_base + tr;
+  if (t < 0 || t >= d.T) return;
+  float* d0 = d.mask + (int64_t)bin * d.T + t;
+  mask_out_pixel<NOUT>(f3, w, offset, n, bin, tr, d0, (int64_t)(f3.H + 1) * d.T, d.T, d.accumulate);
+}
+
+cudaError_t launch_mask_out_many(ActView f3, const float* w, int offset, const WinDesc* wins, cudaStream_t stream) {
+  const int roi = f3.W - 2 * offset;
+  int64_t total = (int64_t)f3.N * f3.H * roi;
+  if (total <= 0) return cudaSuccess;
+  unsigned grid = (unsigned)((total + 255) / 256);
+  switch (f3.C) {
+    case 8: mask_out_many_kernel<8><<<grid, 256, 0, stream>>>(f3, w, offset, wins); break;
+    case 16: mask_out_many_kernel<16><<<grid, 256, 0, stream>>>(f3, w, offset, wins); break;
+    case 32: mask_out_many_kernel<32><<<grid, 256, 0, stream>>>(f3, w, offset, wins); break;
+    case 64: mask_out_many_kernel<64><<<grid, 256, 0, stream>>>(f3, w, offset, wins); break;
+    default: return cudaErrorInvalidValue;
   }
+  return cudaGetLastError();
 }
 
 cudaError_t launch_mask_out(const MaskOutParams& p, cudaStream_t stream) {
@@ -324,9 +394,12 @@ cudaError_t launch_mask_out(const MaskOutParams& p, cudaStream_t stream) {
 }
 
 // ------------------------------------------------------------------------------------------------
-__global__ void absmax_kernel(const float2* __restrict__ spec, int64_t n, float* out) {
+// max|spec[i]| over i = i0, i0 + step, ... < n, reduced over the CTA into *out (atomicMax on the bits: m >= 0).  Every
+// thread of the CTA must call it.
+__device__ __forceinline__ void absmax_block(const float2* __restrict__ spec, int64_t n, int64_t i0, int64_t step,
+                                             float* out) {
   float m = 0.f;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+  for (int64_t i = i0; i < n; i += step) {
     float2 v = spec[i];
     m = fmaxf(m, hypotf(v.x, v.y));
   }
@@ -339,6 +412,10 @@ __global__ void absmax_kernel(const float2* __restrict__ spec, int64_t n, float*
     for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
     if (threadIdx.x == 0) atomicMax(reinterpret_cast<unsigned int*>(out), __float_as_uint(m));  // m >= 0
   }
+}
+
+__global__ void absmax_kernel(const float2* __restrict__ spec, int64_t n, float* out) {
+  absmax_block(spec, n, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x, out);
 }
 
 cudaError_t launch_absmax(const float2* spec, int64_t n, float* out_absmax, cudaStream_t stream) {
@@ -386,9 +463,11 @@ __device__ __forceinline__ float order_unkey(unsigned int k) {
   return __uint_as_float(u);
 }
 
-__global__ void lexmax_kernel(const float2* __restrict__ spec, int64_t n, unsigned long long* scratch) {
+// lexicographic max key of spec[i], i = i0, i0 + step, ... < n, reduced per warp into *scratch
+__device__ __forceinline__ void lexmax_block(const float2* __restrict__ spec, int64_t n, int64_t i0, int64_t step,
+                                             unsigned long long* scratch) {
   unsigned long long best = 0ull;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+  for (int64_t i = i0; i < n; i += step) {
     float2 v = spec[i];
     unsigned long long k = ((unsigned long long)order_key(v.x) << 32) | order_key(v.y);
     best = k > best ? k : best;
@@ -400,14 +479,61 @@ __global__ void lexmax_kernel(const float2* __restrict__ spec, int64_t n, unsign
   if ((threadIdx.x & 31) == 0) atomicMax(scratch, best);
 }
 
-__global__ void lexmax_finish_kernel(const unsigned long long* scratch, float* out_norm) {
-  unsigned long long k = *scratch;
+__device__ __forceinline__ float lexmax_finish(unsigned long long k) {
   float re = order_unkey((unsigned int)(k >> 32));
   float im = order_unkey((unsigned int)(k & 0xffffffffu));
   // the zero padding of X_spec_pad also takes part in the max (inference.py:86-87)
   unsigned long long kz = ((unsigned long long)order_key(0.f) << 32) | order_key(0.f);
   if (kz > k) { re = 0.f; im = 0.f; }
-  *out_norm = hypotf(re, im);
+  return hypotf(re, im);
+}
+
+__global__ void lexmax_kernel(const float2* __restrict__ spec, int64_t n, unsigned long long* scratch) {
+  lexmax_block(spec, n, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x, scratch);
+}
+
+__global__ void lexmax_finish_kernel(const unsigned long long* scratch, float* out_norm) {
+  *out_norm = lexmax_finish(*scratch);
+}
+
+// grid (n_tracks, CTAs per track): CTA (i, j) reduces elements j*256 + tid, strided by gridDim.y*256, of track i
+__global__ void absmax_many_kernel(const NormTrack* __restrict__ tracks, float* out) {
+  const NormTrack tr = tracks[blockIdx.x];
+  absmax_block(tr.spec, tr.n, (int64_t)blockIdx.y * blockDim.x + threadIdx.x, (int64_t)gridDim.y * blockDim.x,
+               out + blockIdx.x);
+}
+
+__global__ void lexmax_many_kernel(const NormTrack* __restrict__ tracks, unsigned long long* scratch) {
+  const NormTrack tr = tracks[blockIdx.x];
+  lexmax_block(tr.spec, tr.n, (int64_t)blockIdx.y * blockDim.x + threadIdx.x, (int64_t)gridDim.y * blockDim.x,
+               scratch + blockIdx.x);
+}
+
+__global__ void lexmax_finish_many_kernel(const unsigned long long* scratch, int n_tracks, float* out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n_tracks) out[i] = lexmax_finish(scratch[i]);
+}
+
+cudaError_t launch_normaliser_many(const NormTrack* tracks, int n_tracks, int64_t max_n, int mode,
+                                   unsigned long long* scratch, float* out, cudaStream_t stream) {
+  if (n_tracks <= 0) return cudaSuccess;
+  cudaError_t e = mode == 0 ? cudaMemsetAsync(out, 0, sizeof(float) * n_tracks, stream)
+                            : cudaMemsetAsync(scratch, 0, sizeof(unsigned long long) * n_tracks, stream);
+  if (e != cudaSuccess) return e;
+  // about as many CTAs in all as the single-track kernels use for one track (148 SMs x 8), at least one per track
+  int64_t per = (max_n + 255) / 256;
+  const int64_t cap = (148 * 8 + n_tracks - 1) / n_tracks;
+  if (per > cap) per = cap;
+  if (per > 65535) per = 65535;
+  if (per < 1) per = 1;
+  dim3 grid((unsigned)n_tracks, (unsigned)per);
+  if (mode == 0) {
+    absmax_many_kernel<<<grid, 256, 0, stream>>>(tracks, out);
+  } else {
+    lexmax_many_kernel<<<grid, 256, 0, stream>>>(tracks, scratch);
+    lexmax_finish_many_kernel<<<(unsigned)((n_tracks + 127) / 128), 128, 0, stream>>>(scratch, n_tracks, out);
+  }
+  return cudaGetLastError();
 }
 
 cudaError_t launch_lexmax_abs(const float2* spec, int64_t n, unsigned long long* scratch, float* out_norm,

@@ -73,6 +73,8 @@ Engine::Engine(const Config& cfg) : cfg_(cfg) {
   cudaEventCreateWithFlags(&ev_join_, cudaEventDisableTiming);
   cudaEventCreateWithFlags(&ev_lstm_fork_, cudaEventDisableTiming);
   cudaEventCreateWithFlags(&ev_lstm_join_, cudaEventDisableTiming);
+  cudaEventCreateWithFlags(&ev_tab_copied_, cudaEventDisableTiming);
+  cudaEventCreateWithFlags(&ev_tab_used_, cudaEventDisableTiming);
 }
 
 Engine::~Engine() {
@@ -82,6 +84,10 @@ Engine::~Engine() {
   if (ws_mask_) cudaFree(ws_mask_);
   if (ws_frames_) cudaFree(ws_frames_);
   if (ws_wave_) cudaFree(ws_wave_);
+  if (ws_norms_) cudaFree(ws_norms_);
+  if (ws_lexs_) cudaFree(ws_lexs_);
+  if (tab_dev_) cudaFree(tab_dev_);
+  if (tab_host_) cudaFreeHost(tab_host_);
   profile_enable(false);
   if (s_hi_) cudaStreamDestroy(s_hi_);
   if (s_copy_) cudaStreamDestroy(s_copy_);
@@ -90,6 +96,8 @@ Engine::~Engine() {
   if (ev_join_) cudaEventDestroy(ev_join_);
   if (ev_lstm_fork_) cudaEventDestroy(ev_lstm_fork_);
   if (ev_lstm_join_) cudaEventDestroy(ev_lstm_join_);
+  if (ev_tab_copied_) cudaEventDestroy(ev_tab_copied_);
+  if (ev_tab_used_) cudaEventDestroy(ev_tab_used_);
 }
 
 bool Engine::load_tensor(const char* name, int dtype, int ndim, const int64_t* shape, const void* data) {
@@ -923,6 +931,219 @@ bool Engine::separate_wave_host(const float* wave, int64_t L, int tta, float* in
     return false;
   }
   return ck(cudaStreamSynchronize(s), "separate_wave_host sync") && ck(cudaStreamSynchronize(s_copy_), "separate_wave_host copy sync");
+}
+
+// ---------------------------------------------------------------------------------------------
+// Several tracks per call.  Windows are independent inside the net (eval-mode BatchNorm, per-sample ASPP pool and
+// LSTM), so windows of different tracks share a forward batch without changing any arithmetic; only the gather into
+// the input buffer, the mask epilogue and the normalisers read per-track tables.
+bool Engine::ensure_norms(int n) {
+  if (n <= ws_norms_cap_) return true;
+  if (ws_norms_) cudaFree(ws_norms_);
+  if (ws_lexs_) cudaFree(ws_lexs_);
+  ws_norms_ = nullptr;
+  ws_lexs_ = nullptr;
+  ws_norms_cap_ = 0;
+  if (!ck(cudaMalloc(&ws_norms_, sizeof(float) * n), "workspace normalisers") ||
+      !ck(cudaMalloc(&ws_lexs_, sizeof(unsigned long long) * n), "workspace lexmax"))
+    return false;
+  ws_norms_cap_ = n;
+  return true;
+}
+
+bool Engine::upload_tables(const Tables& t, cudaStream_t s, const unsigned char** dev) {
+  const size_t nb = t.bytes.size() ? t.bytes.size() : 16;
+  // the previous call's copy out of the pinned buffer must have run before the buffer is rewritten
+  if (!ck(cudaEventSynchronize(ev_tab_copied_), "tables: previous copy")) return false;
+  if (nb > tab_host_cap_) {
+    if (tab_host_) cudaFreeHost(tab_host_);
+    tab_host_ = nullptr;
+    tab_host_cap_ = 0;
+    if (!ck(cudaMallocHost(&tab_host_, nb), "tables: pinned buffer")) return false;
+    tab_host_cap_ = nb;
+  }
+  if (nb > tab_dev_cap_) {
+    if (!ck(cudaEventSynchronize(ev_tab_used_), "tables: previous call")) return false;
+    if (tab_dev_) cudaFree(tab_dev_);
+    tab_dev_ = nullptr;
+    tab_dev_cap_ = 0;
+    if (!ck(cudaMalloc(&tab_dev_, nb), "tables: device buffer")) return false;
+    tab_dev_cap_ = nb;
+  }
+  if (!t.bytes.empty()) memcpy(tab_host_, t.bytes.data(), t.bytes.size());
+  // the previous call's kernels read the device table: the stream waits for them, the host does not
+  if (!ck(cudaStreamWaitEvent(s, ev_tab_used_, 0), "tables: wait") ||
+      !ck(cudaMemcpyAsync(tab_dev_, tab_host_, nb, cudaMemcpyHostToDevice, s), "tables: copy") ||
+      !ck(cudaEventRecord(ev_tab_copied_, s), "tables: record"))
+    return false;
+  *dev = tab_dev_;
+  return true;
+}
+
+// Pass 1 of every track follows make_padding (lib/dataset.py:198-205) as separate() does; with tta, pass 2 of every
+// track uses pad_l + roi/2 and averages into the mask (inference.py:89-98).  All pass-1 windows of all tracks come
+// first, then all pass-2 windows, cut into batches of max_batch.
+//
+// TTA ordering: a pass-2 window averages ((old + new) * 0.5) into mask frames that pass-1 windows of the SAME track
+// wrote.  Within one mask-epilogue launch there is no order between windows, so a batch must never hold a pass-2
+// window of a track together with a pass-1 window of that track: at the pass boundary such a batch is closed early.
+// (Windows of one pass write disjoint frames, and batches run in stream order.)
+void Engine::schedule_windows(const float2* const* specs, const int64_t* T, int n, int tta, float* const* masks,
+                              Schedule& sch) const {
+  const int r = roi(), off = cfg_.offset, B = cfg_.max_batch;
+  sch.wins.clear();
+  sch.chunk_end.clear();
+  for (int pass = 0; pass < (tta ? 2 : 1); ++pass) {
+    for (int i = 0; i < n; ++i) {
+      const int64_t pad_r = r - (T[i] % r) + off;
+      const int64_t Wpad = off + T[i] + pad_r + (pass ? r : 0);   // pass 2: pad_l += roi/2, pad_r += roi/2
+      const int patches = (int)((Wpad - 2 * off) / r);
+      for (int g = 0; g < patches; ++g) {
+        WinDesc d;
+        d.spec = specs[i];
+        d.mask = masks[i];
+        d.T = T[i];
+        d.t_base = (int64_t)g * r - (pass ? r / 2 : 0);
+        d.pad_l = off + (pass ? r / 2 : 0);
+        d.window = g;
+        d.norm = i;
+        d.accumulate = pass;
+        sch.wins.push_back(d);
+      }
+    }
+  }
+  std::vector<char> pass1_in_batch((size_t)n, 0);
+  int start = 0;
+  for (int k = 0; k < (int)sch.wins.size(); ++k) {
+    const WinDesc& d = sch.wins[(size_t)k];
+    if (k - start == B || (d.accumulate && pass1_in_batch[(size_t)d.norm])) {
+      sch.chunk_end.push_back(k);
+      for (int j = start; j < k; ++j) pass1_in_batch[(size_t)sch.wins[(size_t)j].norm] = 0;
+      start = k;
+    }
+    if (!d.accumulate) pass1_in_batch[(size_t)d.norm] = 1;
+  }
+  if (start < (int)sch.wins.size()) sch.chunk_end.push_back((int)sch.wins.size());
+}
+
+// one table-driven pack, the forward and one table-driven mask epilogue per batch; norms in ws_norms_
+bool Engine::run_schedule(const Schedule& sch, const WinDesc* d_wins, cudaStream_t s) {
+  const int max_bin = cfg_.n_fft / 2, nb = bins(), W = cfg_.cropsize, r = roi();
+  int start = 0;
+  for (int end : sch.chunk_end) {
+    const int n_now = end - start;
+    const WinDesc* d = d_wins + start;
+    ++launches;
+    if (!timed("pack_mag_many", n_now, max_bin, W, s, [&] {
+          return ck(launch_pack_mag_many(d, nb, max_bin, W, r, ws_norms_, in3_.view(n_now, 0, max_bin, pos_x_, 2), s), "pack many");
+        }))
+      return false;
+    if (!forward(n_now, s)) return false;
+    ++launches;
+    if (!timed("mask_out_many", n_now, max_bin, W, s, [&] { return ck(launch_mask_out_many(f3_.all(n_now), out_w_, cfg_.offset, d, s), "mask_out many"); }))
+      return false;
+    start = end;
+  }
+  return true;
+}
+
+bool Engine::normalisers_many(const NormTrack* d_tracks, int n, int64_t max_n, int mode, cudaStream_t s) {
+  ++launches;
+  return timed(mode == 0 ? "normaliser.absmax_many" : "normaliser.lexmax_many", n, bins(), 0, s, [&] {
+    return ck(launch_normaliser_many(d_tracks, n, max_n, mode, ws_lexs_, ws_norms_, s), "normalisers");
+  });
+}
+
+bool Engine::separate_many(const float2* const* specs, const int64_t* T, int n, int tta, float* const* masks,
+                           cudaStream_t s) {
+  if (!finalized_) {
+    err = "weights not finalized";
+    return false;
+  }
+  cudaSetDevice(cfg_.device);
+  if (!ensure_norms(n)) return false;
+  std::vector<NormTrack> nt((size_t)n);
+  int64_t max_n = 0;
+  for (int i = 0; i < n; ++i) {
+    nt[(size_t)i].spec = specs[i];
+    nt[(size_t)i].n = (int64_t)2 * bins() * T[i];
+    if (nt[(size_t)i].n > max_n) max_n = nt[(size_t)i].n;
+  }
+  Schedule sch;
+  schedule_windows(specs, T, n, tta, masks, sch);
+  Tables tab;
+  const size_t o_norm = tab.put(nt), o_wins = tab.put(sch.wins);
+  const unsigned char* d = nullptr;
+  if (!upload_tables(tab, s, &d)) return false;
+  if (!normalisers_many((const NormTrack*)(d + o_norm), n, max_n, tta ? 1 : 0, s)) return false;
+  if (!run_schedule(sch, (const WinDesc*)(d + o_wins), s)) return false;
+  return ck(cudaEventRecord(ev_tab_used_, s), "tables: record use");
+}
+
+// waves[i] (2, L[i]) -> inst[i], voc[i] (2, hop*(T_i-1)): ragged STFT into the concatenated spectrogram workspace,
+// per-track normalisers, the packed windows, ragged masked inverse STFT.  One table upload for the whole call.
+bool Engine::separate_waves(const float* const* waves, const int64_t* L, int n, int tta, float* const* inst,
+                            float* const* voc, cudaStream_t s) {
+  if (!finalized_) {
+    err = "weights not finalized";
+    return false;
+  }
+  cudaSetDevice(cfg_.device);
+  const int NF = cfg_.n_fft, hop = cfg_.hop, nb = bins();
+  std::vector<int64_t> T((size_t)n);
+  int64_t sumT = 0;
+  for (int i = 0; i < n; ++i) {
+    T[(size_t)i] = 1 + L[i] / hop;
+    sumT += T[(size_t)i];
+  }
+  if (!ensure_ws(sumT) || !ensure_norms(n)) return false;
+  std::vector<FftTrack> ft((size_t)n);
+  std::vector<NormTrack> nt((size_t)n);
+  std::vector<const float2*> specs((size_t)n);
+  std::vector<float*> masks((size_t)n);
+  int64_t frames = 0, ctas = 0, samples = 0, max_n = 0;
+  for (int i = 0; i < n; ++i) {
+    const int64_t Ti = T[(size_t)i];
+    FftTrack& f = ft[(size_t)i];
+    f.wave = waves[i];
+    f.spec = ws_spec_ + (int64_t)2 * nb * frames;
+    f.mask = ws_mask_ + (int64_t)2 * nb * frames;
+    f.wave_a = inst[i];
+    f.wave_b = voc[i];
+    f.L = L[i];
+    f.T = Ti;
+    f.frame_off = frames;
+    f.cta0 = ctas;
+    f.s0 = samples;
+    frames += Ti;
+    ctas += fft_ctas_per_track(NF, Ti);
+    samples += (int64_t)2 * hop * (Ti - 1);
+    specs[(size_t)i] = f.spec;
+    masks[(size_t)i] = ws_mask_ + (int64_t)2 * nb * f.frame_off;
+    nt[(size_t)i].spec = f.spec;
+    nt[(size_t)i].n = (int64_t)2 * nb * Ti;
+    if (nt[(size_t)i].n > max_n) max_n = nt[(size_t)i].n;
+  }
+  Schedule sch;
+  schedule_windows(specs.data(), T.data(), n, tta, masks.data(), sch);
+  Tables tab;
+  const size_t o_fft = tab.put(ft), o_norm = tab.put(nt), o_wins = tab.put(sch.wins);
+  const unsigned char* d = nullptr;
+  if (!upload_tables(tab, s, &d)) return false;
+  const FftTrack* d_ft = (const FftTrack*)(d + o_fft);
+  ++launches;
+  if (!timed("stft_many", n, nb, (int)frames, s, [&] { return ck(launch_stft_many(d_ft, n, ctas, NF, hop, twiddle_, window_, s), "stft many"); }))
+    return false;
+  if (!normalisers_many((const NormTrack*)(d + o_norm), n, max_n, tta ? 1 : 0, s)) return false;
+  if (!run_schedule(sch, (const WinDesc*)(d + o_wins), s)) return false;
+  float* fa = ws_frames_;
+  float* fb = ws_frames_ + (int64_t)2 * frames * NF;
+  launches += 2;
+  if (!timed("istft.frames_many", n, nb, (int)frames, s, [&] { return ck(launch_istft_frames_many(d_ft, n, ctas, NF, fa, fb, twiddle_, window_, s), "istft frames many"); }))
+    return false;
+  if (!timed("istft.overlap_add_many", n, nb, (int)frames, s, [&] { return ck(launch_istft_ola_many(d_ft, n, samples, NF, hop, fa, fb, window_, s), "istft ola many"); }))
+    return false;
+  return ck(cudaEventRecord(ev_tab_used_, s), "tables: record use");
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <string.h>
 
 #include <functional>
 #include <map>
@@ -127,6 +128,11 @@ class Engine {
   bool separate_wave(const float* wave, int64_t L, int tta, float* inst, float* voc, cudaStream_t s);
   bool separate_wave_host(const float* wave, int64_t L, int tta, float* inst, float* voc, cudaStream_t s);
   bool normaliser(const float2* spec, int64_t T, int mode, float* out, cudaStream_t s);
+  // several tracks per call, their windows packed into shared forward batches (include/vr_b200.h vr_separate_many,
+  // vr_separate_waves); arguments already validated
+  bool separate_many(const float2* const* specs, const int64_t* T, int n, int tta, float* const* masks, cudaStream_t s);
+  bool separate_waves(const float* const* waves, const int64_t* L, int n, int tta, float* const* inst,
+                      float* const* voc, cudaStream_t s);
 
   // debug / tests: run one reference Conv2DBNActiv-shaped layer through a chosen kernel
   bool debug_conv(const float* x_nchw, int N, int Cin, int H, int W, const float* w, const float* bias, int Cout,
@@ -177,6 +183,37 @@ class Engine {
   float* ws_wave_ = nullptr; int64_t ws_wave_cap_ = 0;   // [2][L] in + 2 x [2][Lo] out (host-buffer entry)
   float* ws_norm_ = nullptr;            // [4] floats: absmax, lexmax-abs
   unsigned long long* ws_lex_ = nullptr;
+  // several-track calls: one normaliser (and lexmax scratch) per track, grow-only
+  float* ws_norms_ = nullptr; unsigned long long* ws_lexs_ = nullptr; int64_t ws_norms_cap_ = 0;
+
+  // The tables of a several-track call (window descriptors, track tables) are built on the host, staged in a pinned
+  // buffer and copied to the device once per call, on the call's stream.  The next call may rewrite the pinned buffer
+  // only after that copy has run (ev_tab_copied_, waited on by the host), and the device table only after the previous
+  // call's last reader (ev_tab_used_, waited on by the stream).
+  struct Tables {
+    std::vector<unsigned char> bytes;
+    template <class X>
+    size_t put(const std::vector<X>& v) {
+      const size_t off = (bytes.size() + 15) / 16 * 16;
+      bytes.resize(off + sizeof(X) * v.size());
+      if (!v.empty()) memcpy(bytes.data() + off, v.data(), sizeof(X) * v.size());
+      return off;
+    }
+  };
+  unsigned char* tab_host_ = nullptr; size_t tab_host_cap_ = 0;
+  unsigned char* tab_dev_ = nullptr; size_t tab_dev_cap_ = 0;
+  cudaEvent_t ev_tab_copied_ = nullptr, ev_tab_used_ = nullptr;
+  bool upload_tables(const Tables& t, cudaStream_t s, const unsigned char** dev);
+  // flat window schedule of a several-track call, cut into forward batches: batch b is wins[chunk_end[b-1], chunk_end[b])
+  struct Schedule {
+    std::vector<WinDesc> wins;
+    std::vector<int> chunk_end;
+  };
+  void schedule_windows(const float2* const* specs, const int64_t* T, int n, int tta, float* const* masks,
+                        Schedule& sch) const;
+  bool run_schedule(const Schedule& sch, const WinDesc* d_wins, cudaStream_t s);
+  bool normalisers_many(const NormTrack* d_tracks, int n, int64_t max_n, int mode, cudaStream_t s);
+  bool ensure_norms(int n);
 
   // the high-band BaseNets of stages 1-2 run on their own stream next to the low-band chain (independent until
   // stage 3, lib/nets.py:88-99); disabled while per-kernel profiling is on so event timings stay per-kernel

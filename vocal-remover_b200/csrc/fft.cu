@@ -40,11 +40,10 @@ __device__ __forceinline__ void fft_inplace(float2* z, const float2* __restrict_
   }
 }
 
-__global__ void __launch_bounds__(256) stft_kernel(const float* __restrict__ wave, int64_t L, int NF, int logn,
-                                                   int hop, float2* __restrict__ spec, int64_t T, int64_t t_first,
-                                                   const float2* __restrict__ tw, const float* __restrict__ win) {
-  extern __shared__ float2 z[];
-  const int64_t t = t_first + blockIdx.x;
+// frame t of the track, one CTA, z: NF float2 of shared memory
+__device__ __forceinline__ void stft_frame(const float* __restrict__ wave, int64_t L, int NF, int logn, int hop,
+                                           float2* __restrict__ spec, int64_t T, int64_t t,
+                                           const float2* __restrict__ tw, const float* __restrict__ win, float2* z) {
   const int64_t s0 = t * hop - NF / 2;
   for (int n = threadIdx.x; n < NF; n += blockDim.x) {
     const int64_t s = s0 + n;
@@ -65,6 +64,24 @@ __global__ void __launch_bounds__(256) stft_kernel(const float* __restrict__ wav
     spec[((int64_t)0 * bins + k) * T + t] = make_float2(0.5f * (a.x + b.x), 0.5f * (a.y - b.y));
     spec[((int64_t)1 * bins + k) * T + t] = make_float2(0.5f * (a.y + b.y), -0.5f * (a.x - b.x));
   }
+}
+
+__global__ void __launch_bounds__(256) stft_kernel(const float* __restrict__ wave, int64_t L, int NF, int logn,
+                                                   int hop, float2* __restrict__ spec, int64_t T, int64_t t_first,
+                                                   const float2* __restrict__ tw, const float* __restrict__ win) {
+  extern __shared__ float2 z[];
+  stft_frame(wave, L, NF, logn, hop, spec, T, t_first + blockIdx.x, tw, win, z);
+}
+
+// index of the track whose [first, next first) range holds x (tracks sorted by first, tracks[0].first == 0)
+template <int64_t FftTrack::*FIRST>
+__device__ __forceinline__ int find_track(const FftTrack* __restrict__ tracks, int n_tracks, int64_t x) {
+  int lo = 0, hi = n_tracks - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (tracks[mid].*FIRST <= x) lo = mid; else hi = mid - 1;
+  }
+  return lo;
 }
 
 
@@ -179,12 +196,11 @@ __device__ __forceinline__ void fft2048_frames(float2* z, const float2* __restri
   __syncthreads();
 }
 
-__global__ void __launch_bounds__(256) stft2048_kernel(const float* __restrict__ wave, int64_t L, int hop,
-                                                       float2* __restrict__ spec, int64_t T, int64_t t_first, int64_t t_end,
-                                                       const float2* __restrict__ tw, const float* __restrict__ win) {
-  extern __shared__ float2 z[];
+// frames [t0, min(t0 + kFR, t_end)) of the track, one CTA
+__device__ __forceinline__ void stft2048_frames(const float* __restrict__ wave, int64_t L, int hop,
+                                                float2* __restrict__ spec, int64_t T, int64_t t0, int64_t t_end,
+                                                const float2* __restrict__ tw, const float* __restrict__ win, float2* z) {
   constexpr int NF = kF2048;
-  const int64_t t0 = t_first + (int64_t)blockIdx.x * kFR;
   for (int f = 0; f < kFR; ++f) {
     const int64_t s0 = (t0 + f) * hop - NF / 2;
     float2* zf = z + f * kFrameSlots;
@@ -230,19 +246,23 @@ __global__ void __launch_bounds__(256) stft2048_kernel(const float* __restrict__
   }
 }
 
-// grid (ceil(nfr / kFR), 2 channels).  Inverse transform through the forward one: ifft(x) = conj(fft(conj(x))).
-__global__ void __launch_bounds__(256) istft2048_frames_kernel(const float2* __restrict__ spec,
-                                                               const float* __restrict__ mask, int64_t T, int64_t t_first,
-                                                               int64_t nfr, float* __restrict__ frames_a,
-                                                               float* __restrict__ frames_b,
-                                                               const float2* __restrict__ tw,
-                                                               const float* __restrict__ win) {
+__global__ void __launch_bounds__(256) stft2048_kernel(const float* __restrict__ wave, int64_t L, int hop,
+                                                       float2* __restrict__ spec, int64_t T, int64_t t_first, int64_t t_end,
+                                                       const float2* __restrict__ tw, const float* __restrict__ win) {
   extern __shared__ float2 z[];
+  stft2048_frames(wave, L, hop, spec, T, t_first + (int64_t)blockIdx.x * kFR, t_end, tw, win, z);
+}
+
+// Inverse transform through the forward one: ifft(x) = conj(fft(conj(x))).  Channel c, scratch frames
+// [fr0, min(fr0 + kFR, nfr)) = track frames t_first + fr0 ..., one CTA.
+__device__ __forceinline__ void istft2048_frames(const float2* __restrict__ spec, const float* __restrict__ mask,
+                                                 int64_t T, int64_t t_first, int64_t nfr, int64_t fr0, int c,
+                                                 float* __restrict__ frames_a, float* __restrict__ frames_b,
+                                                 const float2* __restrict__ tw, const float* __restrict__ win,
+                                                 float2* z) {
   constexpr int NF = kF2048;
   constexpr int bins = NF / 2 + 1;
-  const int64_t fr0 = (int64_t)blockIdx.x * kFR;   // first frame of this CTA inside the scratch
   const int64_t t0 = t_first + fr0;
-  const int c = blockIdx.y;
   const int nf = (int)(nfr - fr0 < kFR ? nfr - fr0 : kFR);
   for (int k = threadIdx.x; k < bins; k += blockDim.x) {
     const int64_t gi = ((int64_t)c * bins + k) * T + t0;
@@ -286,6 +306,40 @@ __global__ void __launch_bounds__(256) istft2048_frames_kernel(const float2* __r
   }
 }
 
+// grid (ceil(nfr / kFR), 2 channels)
+__global__ void __launch_bounds__(256) istft2048_frames_kernel(const float2* __restrict__ spec,
+                                                               const float* __restrict__ mask, int64_t T, int64_t t_first,
+                                                               int64_t nfr, float* __restrict__ frames_a,
+                                                               float* __restrict__ frames_b,
+                                                               const float2* __restrict__ tw,
+                                                               const float* __restrict__ win) {
+  extern __shared__ float2 z[];
+  istft2048_frames(spec, mask, T, t_first, nfr, (int64_t)blockIdx.x * kFR, blockIdx.y, frames_a, frames_b, tw, win, z);
+}
+
+// ---- several tracks per launch: grid (total CTAs, 2 channels for the inverse) ----
+__global__ void __launch_bounds__(256) stft2048_many_kernel(const FftTrack* __restrict__ tracks, int n_tracks, int hop,
+                                                            const float2* __restrict__ tw,
+                                                            const float* __restrict__ win) {
+  extern __shared__ float2 z[];
+  const int i = find_track<&FftTrack::cta0>(tracks, n_tracks, blockIdx.x);
+  const FftTrack& tr = tracks[i];
+  stft2048_frames(tr.wave, tr.L, hop, tr.spec, tr.T, ((int64_t)blockIdx.x - tr.cta0) * kFR, tr.T, tw, win, z);
+}
+
+__global__ void __launch_bounds__(256) istft2048_frames_many_kernel(const FftTrack* __restrict__ tracks, int n_tracks,
+                                                                    float* __restrict__ frames_a,
+                                                                    float* __restrict__ frames_b,
+                                                                    const float2* __restrict__ tw,
+                                                                    const float* __restrict__ win) {
+  extern __shared__ float2 z[];
+  const int i = find_track<&FftTrack::cta0>(tracks, n_tracks, blockIdx.x);
+  const FftTrack& tr = tracks[i];
+  const int64_t off = 2 * tr.frame_off * kF2048;
+  istft2048_frames(tr.spec, tr.mask, tr.T, 0, tr.T, ((int64_t)blockIdx.x - tr.cta0) * kFR, blockIdx.y, frames_a + off,
+                   frames_b ? frames_b + off : nullptr, tw, win, z);
+}
+
 static constexpr size_t kSmem2048 = (size_t)kFR * kFrameSlots * sizeof(float2);   // 73,728 bytes
 
 static bool fft2048_ready() {   // per-device opt-in to more than 48 KB of dynamic shared memory
@@ -295,7 +349,11 @@ static bool fft2048_ready() {   // per-device opt-in to more than 48 KB of dynam
   if (!done[dev]) {
     if (cudaFuncSetAttribute(stft2048_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem2048) != cudaSuccess ||
         cudaFuncSetAttribute(istft2048_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem2048) !=
-            cudaSuccess)
+            cudaSuccess ||
+        cudaFuncSetAttribute(stft2048_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem2048) !=
+            cudaSuccess ||
+        cudaFuncSetAttribute(istft2048_frames_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)kSmem2048) != cudaSuccess)
       return false;
     done[dev] = true;
   }
@@ -318,17 +376,11 @@ cudaError_t launch_stft(const float* wave, int64_t L, int n_fft, int hop, float2
   return cudaGetLastError();
 }
 
-// grid (T, 2 channels): windowed inverse transform of one frame of one channel -> frames[stem][c][t][NF]
-__global__ void __launch_bounds__(256) istft_frames_kernel(const float2* __restrict__ spec,
-                                                           const float* __restrict__ mask, int NF, int logn,
-                                                           int64_t T, int64_t t_first, int64_t nfr,
-                                                           float* __restrict__ frames_a,
-                                                           float* __restrict__ frames_b,
-                                                           const float2* __restrict__ tw,
-                                                           const float* __restrict__ win) {
-  extern __shared__ float2 z[];
-  const int64_t t = t_first + blockIdx.x;
-  const int c = blockIdx.y;
+// Windowed inverse transform of frame t of channel c -> fa (and fb) [NF], one CTA, z: NF float2 of shared memory
+__device__ __forceinline__ void istft_frame(const float2* __restrict__ spec, const float* __restrict__ mask, int NF,
+                                            int logn, int64_t T, int64_t t, int c, float* __restrict__ fa,
+                                            float* __restrict__ fb, const float2* __restrict__ tw,
+                                            const float* __restrict__ win, float2* z) {
   const int bins = NF / 2 + 1;
   for (int k = threadIdx.x; k < bins; k += blockDim.x) {
     const int64_t gi = ((int64_t)c * bins + k) * T + t;
@@ -357,8 +409,6 @@ __global__ void __launch_bounds__(256) istft_frames_kernel(const float2* __restr
   __syncthreads();
   fft_inplace<true>(z, tw, NF, logn);
   const float inv = 1.f / (float)NF;
-  float* fa = frames_a + ((int64_t)c * nfr + blockIdx.x) * NF;
-  float* fb = frames_b ? frames_b + ((int64_t)c * nfr + blockIdx.x) * NF : nullptr;
   for (int n = threadIdx.x; n < NF; n += blockDim.x) {
     const float w = win[n] * inv;
     fa[n] = z[n].x * w;
@@ -366,16 +416,26 @@ __global__ void __launch_bounds__(256) istft_frames_kernel(const float2* __restr
   }
 }
 
-// Output samples [s0, s1) of each channel; the scratch holds frames [t_first, t_first + nfr) of the track.
-__global__ void istft_ola_kernel(const float* __restrict__ frames_a, const float* __restrict__ frames_b, int NF,
-                                 int hop, int64_t T, int64_t t_first, int64_t nfr, int64_t s0, int64_t s1, int64_t Lo,
-                                 float* __restrict__ wave_a, float* __restrict__ wave_b,
-                                 const float* __restrict__ win) {
-  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t span = s1 - s0;
-  if (idx >= 2 * span) return;
-  const int c = (int)(idx / span);
-  const int64_t s = s0 + idx % span;
+// grid (T, 2 channels): windowed inverse transform of one frame of one channel -> frames[stem][c][t][NF]
+__global__ void __launch_bounds__(256) istft_frames_kernel(const float2* __restrict__ spec,
+                                                           const float* __restrict__ mask, int NF, int logn,
+                                                           int64_t T, int64_t t_first, int64_t nfr,
+                                                           float* __restrict__ frames_a,
+                                                           float* __restrict__ frames_b,
+                                                           const float2* __restrict__ tw,
+                                                           const float* __restrict__ win) {
+  extern __shared__ float2 z[];
+  const int c = blockIdx.y;
+  float* fa = frames_a + ((int64_t)c * nfr + blockIdx.x) * NF;
+  float* fb = frames_b ? frames_b + ((int64_t)c * nfr + blockIdx.x) * NF : nullptr;
+  istft_frame(spec, mask, NF, logn, T, t_first + blockIdx.x, c, fa, fb, tw, win, z);
+}
+
+// Output sample s of channel c; the scratch holds frames [t_first, t_first + nfr) of the track.
+__device__ __forceinline__ void istft_ola_sample(const float* __restrict__ frames_a, const float* __restrict__ frames_b,
+                                                 int NF, int hop, int64_t T, int64_t t_first, int64_t nfr, int64_t Lo,
+                                                 int c, int64_t s, float* __restrict__ wave_a,
+                                                 float* __restrict__ wave_b, const float* __restrict__ win) {
   const int64_t u = s + NF / 2;
   int64_t t1 = u / hop;
   if (t1 > T - 1) t1 = T - 1;
@@ -396,6 +456,52 @@ __global__ void istft_ola_kernel(const float* __restrict__ frames_a, const float
   }
   wave_a[(int64_t)c * Lo + s] = acc_a;
   if (wave_b) wave_b[(int64_t)c * Lo + s] = acc_b;
+}
+
+// Output samples [s0, s1) of each channel; the scratch holds frames [t_first, t_first + nfr) of the track.
+__global__ void istft_ola_kernel(const float* __restrict__ frames_a, const float* __restrict__ frames_b, int NF,
+                                 int hop, int64_t T, int64_t t_first, int64_t nfr, int64_t s0, int64_t s1, int64_t Lo,
+                                 float* __restrict__ wave_a, float* __restrict__ wave_b,
+                                 const float* __restrict__ win) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t span = s1 - s0;
+  if (idx >= 2 * span) return;
+  istft_ola_sample(frames_a, frames_b, NF, hop, T, t_first, nfr, Lo, (int)(idx / span), s0 + idx % span, wave_a, wave_b,
+                   win);
+}
+
+// ---- several tracks per launch (radix-2 frames for n_fft != 2048, overlap-add for every n_fft) ----
+__global__ void __launch_bounds__(256) stft_many_kernel(const FftTrack* __restrict__ tracks, int n_tracks, int NF,
+                                                        int logn, int hop, const float2* __restrict__ tw,
+                                                        const float* __restrict__ win) {
+  extern __shared__ float2 z[];
+  const FftTrack& tr = tracks[find_track<&FftTrack::cta0>(tracks, n_tracks, blockIdx.x)];
+  stft_frame(tr.wave, tr.L, NF, logn, hop, tr.spec, tr.T, (int64_t)blockIdx.x - tr.cta0, tw, win, z);
+}
+
+__global__ void __launch_bounds__(256) istft_frames_many_kernel(const FftTrack* __restrict__ tracks, int n_tracks,
+                                                                int NF, int logn, float* __restrict__ frames_a,
+                                                                float* __restrict__ frames_b,
+                                                                const float2* __restrict__ tw,
+                                                                const float* __restrict__ win) {
+  extern __shared__ float2 z[];
+  const FftTrack& tr = tracks[find_track<&FftTrack::cta0>(tracks, n_tracks, blockIdx.x)];
+  const int c = blockIdx.y;
+  const int64_t t = (int64_t)blockIdx.x - tr.cta0;
+  const int64_t fi = (2 * tr.frame_off + (int64_t)c * tr.T + t) * NF;
+  istft_frame(tr.spec, tr.mask, NF, logn, tr.T, t, c, frames_a + fi, frames_b ? frames_b + fi : nullptr, tw, win, z);
+}
+
+__global__ void istft_ola_many_kernel(const FftTrack* __restrict__ tracks, int n_tracks, int64_t total, int NF, int hop,
+                                      const float* __restrict__ frames_a, const float* __restrict__ frames_b,
+                                      const float* __restrict__ win) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= total) return;
+  const FftTrack& tr = tracks[find_track<&FftTrack::s0>(tracks, n_tracks, idx)];
+  const int64_t Lo = (int64_t)hop * (tr.T - 1), local = idx - tr.s0;
+  const int64_t off = 2 * tr.frame_off * NF;
+  istft_ola_sample(frames_a + off, frames_b ? frames_b + off : nullptr, NF, hop, tr.T, 0, tr.T, Lo, (int)(local / Lo),
+                   local % Lo, tr.wave_a, tr.wave_b, win);
 }
 
 // frames scratch is provided by the caller through wave-independent workspace (see engine.cu)
@@ -425,6 +531,55 @@ cudaError_t launch_istft_ola(const float* frames_a, const float* frames_b, int n
   if (s1 <= s0) return cudaSuccess;
   istft_ola_kernel<<<(unsigned)((2 * (s1 - s0) + 255) / 256), 256, 0, stream>>>(frames_a, frames_b, n_fft, hop, T, t_first,
                                                                                 nfr, s0, s1, Lo, wave_a, wave_b, window);
+  return cudaGetLastError();
+}
+
+// The n_fft = 2048 kernels take kFR frames per CTA, the radix-2 kernels one.
+int64_t fft_ctas_per_track(int n_fft, int64_t T) { return n_fft == kF2048 ? (T + kFR - 1) / kFR : T; }
+
+static bool fft_logn(int n_fft, int& logn) {
+  logn = 0;
+  while ((1 << logn) < n_fft) ++logn;
+  return (1 << logn) == n_fft && n_fft <= 4096 && n_fft >= 64;
+}
+
+cudaError_t launch_stft_many(const FftTrack* tracks, int n_tracks, int64_t total_ctas, int n_fft, int hop,
+                             const float2* twiddle, const float* window, cudaStream_t stream) {
+  int logn;
+  if (!fft_logn(n_fft, logn)) return cudaErrorInvalidValue;
+  if (total_ctas <= 0) return cudaSuccess;
+  if (n_fft == kF2048) {
+    if (!fft2048_ready()) return cudaErrorInvalidValue;
+    stft2048_many_kernel<<<(unsigned)total_ctas, 256, kSmem2048, stream>>>(tracks, n_tracks, hop, twiddle, window);
+  } else {
+    stft_many_kernel<<<(unsigned)total_ctas, 256, n_fft * sizeof(float2), stream>>>(tracks, n_tracks, n_fft, logn, hop,
+                                                                                    twiddle, window);
+  }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_istft_frames_many(const FftTrack* tracks, int n_tracks, int64_t total_ctas, int n_fft, float* frames_a,
+                                     float* frames_b, const float2* twiddle, const float* window, cudaStream_t stream) {
+  int logn;
+  if (!fft_logn(n_fft, logn)) return cudaErrorInvalidValue;
+  if (total_ctas <= 0) return cudaSuccess;
+  dim3 grid((unsigned)total_ctas, 2);
+  if (n_fft == kF2048) {
+    if (!fft2048_ready()) return cudaErrorInvalidValue;
+    istft2048_frames_many_kernel<<<grid, 256, kSmem2048, stream>>>(tracks, n_tracks, frames_a, frames_b, twiddle, window);
+  } else {
+    istft_frames_many_kernel<<<grid, 256, n_fft * sizeof(float2), stream>>>(tracks, n_tracks, n_fft, logn, frames_a,
+                                                                            frames_b, twiddle, window);
+  }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_istft_ola_many(const FftTrack* tracks, int n_tracks, int64_t total_samples, int n_fft, int hop,
+                                  const float* frames_a, const float* frames_b, const float* window, cudaStream_t stream) {
+  if (total_samples <= 0) return cudaSuccess;
+  istft_ola_many_kernel<<<(unsigned)((total_samples + 255) / 256), 256, 0, stream>>>(tracks, n_tracks, total_samples,
+                                                                                    n_fft, hop, frames_a, frames_b,
+                                                                                    window);
   return cudaGetLastError();
 }
 

@@ -39,6 +39,30 @@ struct MaskOutParams {
 };
 cudaError_t launch_mask_out(const MaskOutParams& p, cudaStream_t stream);
 
+// ---- several tracks per launch (vr_separate_many / vr_separate_waves) -----------------------------------------
+// One window of a packed forward batch: batch slot n reads wins[n].  Pack: |X|/norms[norm] of window `window` of the
+// spectrogram spec [2][bins][T] padded by pad_l zeros on the left.  Mask epilogue: kept frame tr of the window goes to
+// mask[c][bin][t_base + tr] (mask [2][bins][T]) if that lies in [0, T); accumulate = 1 averages with what is there.
+struct WinDesc {
+  const float2* spec;
+  float* mask;
+  int64_t T;
+  int64_t t_base;
+  int pad_l, window, norm, accumulate;
+};
+cudaError_t launch_pack_mag_many(const WinDesc* wins, int bins, int max_bin, int W, int roi, const float* norms,
+                                 ActView dst, cudaStream_t stream);
+cudaError_t launch_mask_out_many(ActView f3, const float* w, int offset, const WinDesc* wins, cudaStream_t stream);
+// normaliser of each track: spec with n complex elements -> out[track]
+struct NormTrack {
+  const float2* spec;
+  int64_t n;
+};
+// mode 0: max|X| (launch_absmax), 1: |lexicographic max| with the zero padding taking part (launch_lexmax_abs);
+// scratch: n_tracks entries; max_n: largest n of the table (sizes the grid)
+cudaError_t launch_normaliser_many(const NormTrack* tracks, int n_tracks, int64_t max_n, int mode,
+                                   unsigned long long* scratch, float* out, cudaStream_t stream);
+
 cudaError_t launch_absmax(const float2* spec, int64_t n, float* out_absmax, cudaStream_t stream);
 // max |spec[r][t]| over rows r < nrows and frames t in [t0, t1) of a [nrows][T] array
 cudaError_t launch_absmax_range(const float2* spec, int nrows, int64_t T, int64_t t0, int64_t t1, float* out_absmax,
@@ -82,6 +106,30 @@ cudaError_t launch_istft_frames(const float2* spec, const float* mask, int n_fft
 cudaError_t launch_istft_ola(const float* frames_a, const float* frames_b, int n_fft, int hop, int64_t T,
                              int64_t t_first, int64_t nfr, int64_t s0, int64_t s1, float* wave_a, float* wave_b,
                              const float* window, cudaStream_t stream);
+
+// Ragged forms over several tracks, one launch each.  A track's CTAs (STFT, iSTFT frames: cta0) and its output samples
+// (overlap-add: s0, 2 * hop * (T-1) per track) start at prefix sums of the earlier tracks' counts, ascending; a CTA or
+// thread finds its track by binary search.  The iSTFT frames of track i sit at frames_a / frames_b + 2 * frame_off *
+// n_fft, laid out [c][T][n_fft] as launch_istft_frames writes them.
+struct FftTrack {
+  const float* wave;   // STFT input [2][L]
+  float2* spec;        // [2][bins][T] (iSTFT: read)
+  const float* mask;   // iSTFT: [2][bins][T]
+  float* wave_a;       // iSTFT outputs [2][hop*(T-1)]
+  float* wave_b;
+  int64_t L, T;
+  int64_t frame_off;   // sum of the earlier tracks' T
+  int64_t cta0;        // first CTA of the track in launch_stft_many / launch_istft_frames_many
+  int64_t s0;          // first output sample of the track in launch_istft_ola_many
+};
+// CTAs a track of T frames takes in launch_stft_many / launch_istft_frames_many (the same count for both)
+int64_t fft_ctas_per_track(int n_fft, int64_t T);
+cudaError_t launch_stft_many(const FftTrack* tracks, int n_tracks, int64_t total_ctas, int n_fft, int hop,
+                             const float2* twiddle, const float* window, cudaStream_t stream);
+cudaError_t launch_istft_frames_many(const FftTrack* tracks, int n_tracks, int64_t total_ctas, int n_fft, float* frames_a,
+                                     float* frames_b, const float2* twiddle, const float* window, cudaStream_t stream);
+cudaError_t launch_istft_ola_many(const FftTrack* tracks, int n_tracks, int64_t total_samples, int n_fft, int hop,
+                                  const float* frames_a, const float* frames_b, const float* window, cudaStream_t stream);
 
 // ---- sample-rate conversion (resample.cu), resampy.resample(filter='kaiser_fast') behind librosa.load ----------
 // x [C][n_in] -> y [C][n_out], n_out = int(n_in * sample_ratio); win / delta: the (ratio-scaled) half filter table and

@@ -52,15 +52,33 @@ class Separator(object):
         ctx.check(ctx.lib.vr_separate(ctx.handle, _native.ptr(d_spec), T, 1 if tta else 0, _native.ptr(d_mask),
                                       _native.stream_ptr()), 'vr_separate')
         if self.postprocess:
-            # --postprocess (inference.py:27-30): only T floats leave the device, the run detection of
-            # merge_artifacts runs on the host, the fade weights are applied on the device
-            frame_min = torch.empty(T, dtype=torch.float32, device=d_spec.device)
-            ctx.check(ctx.lib.vr_mask_frame_min(ctx.handle, _native.ptr(d_mask), T, _native.ptr(frame_min),
-                                                _native.stream_ptr()), 'vr_mask_frame_min')
-            weight = torch.from_numpy(spec_utils.artifact_weights(frame_min.cpu().numpy())).to(d_spec.device)
-            ctx.check(ctx.lib.vr_mask_apply_weight(ctx.handle, _native.ptr(d_mask), T, _native.ptr(weight),
-                                                   _native.stream_ptr()), 'vr_mask_apply_weight')
+            self._postprocess_device(d_mask)
         return d_mask
+
+    def _masks_device(self, d_specs, tta):
+        """Masks of several device spectrograms (2, bins, T_i), one per track, with the windows of all tracks packed
+        into shared forward batches (vr_separate_many); each equals what _mask_device gives for that track alone."""
+        ctx = self._ctx()
+        d_masks = [torch.empty((2, s.shape[1], s.shape[2]), dtype=torch.float32, device=s.device) for s in d_specs]
+        ctx.check(ctx.lib.vr_separate_many(ctx.handle, len(d_specs), _native.ptr_array(d_specs),
+                                           _native.i64_array([s.shape[2] for s in d_specs]), 1 if tta else 0,
+                                           _native.ptr_array(d_masks), _native.stream_ptr()), 'vr_separate_many')
+        if self.postprocess:
+            for d_mask in d_masks:
+                self._postprocess_device(d_mask)
+        return d_masks
+
+    def _postprocess_device(self, d_mask):
+        # --postprocess (inference.py:27-30): only T floats leave the device, the run detection of
+        # merge_artifacts runs on the host, the fade weights are applied on the device
+        ctx = self._ctx()
+        T = d_mask.shape[2]
+        frame_min = torch.empty(T, dtype=torch.float32, device=d_mask.device)
+        ctx.check(ctx.lib.vr_mask_frame_min(ctx.handle, _native.ptr(d_mask), T, _native.ptr(frame_min),
+                                            _native.stream_ptr()), 'vr_mask_frame_min')
+        weight = torch.from_numpy(spec_utils.artifact_weights(frame_min.cpu().numpy())).to(d_mask.device)
+        ctx.check(ctx.lib.vr_mask_apply_weight(ctx.handle, _native.ptr(d_mask), T, _native.ptr(weight),
+                                               _native.stream_ptr()), 'vr_mask_apply_weight')
 
     def _run(self, X_spec, tta):
         X_spec = self._check_spec(X_spec)
@@ -149,16 +167,107 @@ class Separator(object):
                                                     voc.ctypes.data, _native.stream_ptr()), 'vr_separate_wave_host')
             return inst, voc
 
+    def separate_waves(self, waves, tta=False):
+        """Several float32 (2, L_i) waves -> a list of (instruments, vocals), one per wave, each what separate_wave
+        gives for that wave alone.  The windows of all tracks share the forward batches of ``batchsize`` windows, so
+        short clips and the partial last batch of every track do not each pay for a nearly empty forward.  Numpy
+        waves give numpy stems, CUDA tensors give CUDA tensors."""
+        ctx = self._ctx()
+        dev = self._dev()
+        hop, n_fft = self.model.hop_length, self.model.n_fft
+        with torch.cuda.device(dev):
+            host = [not (torch.is_tensor(w) and w.is_cuda) for w in waves]
+            d_waves = [torch.from_numpy(np.ascontiguousarray(np.asarray(w, dtype=np.float32))).to(dev) if h
+                       else w.contiguous().float() for w, h in zip(waves, host)]
+            for w in d_waves:
+                if w.dim() != 2 or w.shape[0] != 2:
+                    raise ValueError('every wave must have shape (2, L)')
+            Ts = [1 + w.shape[1] // hop for w in d_waves]
+            inst = [_device_empty((2, hop * (T - 1)), dev) for T in Ts]
+            voc = [_device_empty((2, hop * (T - 1)), dev) for T in Ts]
+            if self.postprocess:
+                # staged on the device: per-track STFT -> packed masks (+ postprocess) -> per-track masked inverse STFT
+                d_specs = []
+                for w, T in zip(d_waves, Ts):
+                    d_spec = torch.empty((2, n_fft // 2 + 1, T), dtype=torch.complex64, device=dev)
+                    ctx.check(ctx.lib.vr_stft(ctx.handle, _native.ptr(w), w.shape[1], _native.ptr(d_spec), T, None,
+                                              _native.stream_ptr()), 'vr_stft')
+                    d_specs.append(d_spec)
+                d_masks = self._masks_device(d_specs, tta)
+                for d_spec, d_mask, a, b in zip(d_specs, d_masks, inst, voc):
+                    ctx.check(ctx.lib.vr_apply_mask_istft(ctx.handle, _native.ptr(d_spec), _native.ptr(d_mask),
+                                                          d_spec.shape[2], _native.ptr(a), _native.ptr(b),
+                                                          _native.stream_ptr()), 'vr_apply_mask_istft')
+            else:
+                ctx.check(ctx.lib.vr_separate_waves(ctx.handle, len(d_waves), _native.ptr_array(d_waves),
+                                                    _native.i64_array([w.shape[1] for w in d_waves]), 1 if tta else 0,
+                                                    _native.ptr_array(inst), _native.ptr_array(voc),
+                                                    _native.stream_ptr()), 'vr_separate_waves')
+            return [(a.cpu().numpy(), b.cpu().numpy()) if h else (a, b) for a, b, h in zip(inst, voc, host)]
+
+
+def _device_empty(shape, dev):
+    """float32 tensor of `shape` whose data pointer is never NULL (a zero-size tensor has no storage, and the native
+    calls reject NULL pointers): one spare element is allocated behind it."""
+    n = int(np.prod(shape))
+    return torch.empty(n + 1, dtype=torch.float32, device=dev)[:n].view(shape)
+
 
 MODEL_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'models')
 DEFAULT_MODEL_PATH = os.path.join(MODEL_DIR, 'baseline.pth')
+# Audio per separate_waves call when several inputs are given: the workspaces grow with the call's total frame count,
+# and 2400 s is the 40-minute stream bench.py already runs on one GPU.
+GROUP_SECONDS = 2400.0
+
+
+def _basename(path):
+    return os.path.splitext(os.path.basename(path))[0]
+
+
+def group_by_seconds(items, seconds_of, budget=GROUP_SECONDS):
+    """Consecutive items in groups of at most `budget` seconds of audio; an item longer than that is a group alone.
+    `items` is consumed lazily, so only one group (and the item that closes it) is held at a time."""
+    group, total = [], 0.0
+    for item in items:
+        sec = seconds_of(item)
+        if group and total + sec > budget:
+            yield group
+            group, total = [], 0.0
+        group.append(item)
+        total += sec
+    if group:
+        yield group
+
+
+def _separate_files(sp, paths, args, device, output_dir):
+    """Several inputs with one loaded model: each group of inputs is one separate_waves call."""
+    def load_all():
+        for path in paths:
+            print('loading wave source {}...'.format(path), end=' ')
+            X, sr = audio_io.load(path, sr=args.sr, mono=False, dtype=np.float32, device=device)
+            print('done')
+            if X.ndim == 1:
+                # mono to stereo
+                X = np.asarray([X, X])
+            yield path, X, sr
+
+    for group in group_by_seconds(load_all(), lambda item: item[1].shape[-1] / float(item[2])):
+        print('stft of {} wave sources, separation, inverse stft of instruments and vocals...'.format(len(group)),
+              end=' ')
+        stems = sp.separate_waves([X for _, X, _ in group], tta=args.tta)
+        print('done')
+        writer = audio_io.AsyncWriter()
+        for (path, _, sr), (wave_inst, wave_voc) in zip(group, stems):
+            writer.write('{}{}_Instruments.wav'.format(output_dir, _basename(path)), wave_inst.T, sr)
+            writer.write('{}{}_Vocals.wav'.format(output_dir, _basename(path)), wave_voc.T, sr)
+        writer.join()
 
 
 def main():
     p = argparse.ArgumentParser()
     p.add_argument('--gpu', '-g', type=int, default=-1)
     p.add_argument('--pretrained_model', '-P', type=str, default=DEFAULT_MODEL_PATH)
-    p.add_argument('--input', '-i', required=True)
+    p.add_argument('--input', '-i', required=True, nargs='+')
     p.add_argument('--sr', '-r', type=int, default=44100)
     p.add_argument('--n_fft', '-f', type=int, default=2048)
     p.add_argument('--hop_length', '-H', type=int, default=1024)
@@ -169,6 +278,11 @@ def main():
     p.add_argument('--postprocess', '-p', action='store_true')
     p.add_argument('--output_dir', '-o', type=str, default="")
     args = p.parse_args()
+    # several inputs write <basename>_Instruments.wav / _Vocals.wav each: two with the same basename would overwrite
+    names = [_basename(path) for path in args.input]
+    dup = sorted(set(n for n in names if names.count(n) > 1))
+    if dup:
+        p.error('inputs with the same basename would overwrite each other\'s output files: {}'.format(', '.join(dup)))
 
     # unsupported surfaces fail before any heavy work (model load, audio decode, output directory)
     if args.output_image:
@@ -187,9 +301,19 @@ def main():
     spec_utils.set_device(device.index)
     print('done')
 
+    if len(args.input) > 1:
+        sp = Separator(model=model, device=device, batchsize=args.batchsize, cropsize=args.cropsize,
+                       postprocess=args.postprocess)
+        output_dir = args.output_dir
+        if output_dir != "":
+            output_dir = output_dir.rstrip('/') + '/'
+            os.makedirs(output_dir, exist_ok=True)
+        _separate_files(sp, args.input, args, device, output_dir)
+        return
+
     print('loading wave source...', end=' ')
-    X, sr = audio_io.load(args.input, sr=args.sr, mono=False, dtype=np.float32, device=device)
-    basename = os.path.splitext(os.path.basename(args.input))[0]
+    X, sr = audio_io.load(args.input[0], sr=args.sr, mono=False, dtype=np.float32, device=device)
+    basename = os.path.splitext(os.path.basename(args.input[0]))[0]
     print('done')
 
     if X.ndim == 1:

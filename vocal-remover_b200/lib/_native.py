@@ -43,6 +43,10 @@ SIGNATURES = {
     'vr_apply_mask_istft_range': (c_i32, [c_vp, c_vp, c_fp, c_i64, c_i64, c_i64, c_fp, c_fp, c_vp]),
     'vr_separate_wave': (c_i32, [c_vp, c_fp, c_i64, c_i32, c_fp, c_fp, c_vp]),
     'vr_separate_wave_host': (c_i32, [c_vp, c_fp, c_i64, c_i32, c_fp, c_fp, c_vp]),
+    'vr_separate_many': (c_i32, [c_vp, c_i32, ctypes.POINTER(c_vp), ctypes.POINTER(c_i64), c_i32,
+                                 ctypes.POINTER(c_vp), c_vp]),
+    'vr_separate_waves': (c_i32, [c_vp, c_i32, ctypes.POINTER(c_vp), ctypes.POINTER(c_i64), c_i32,
+                                  ctypes.POINTER(c_vp), ctypes.POINTER(c_vp), c_vp]),
     'vr_shared_alloc': (c_i32, [c_vp, c_i64, ctypes.POINTER(c_vp), ctypes.c_char_p]),
     'vr_shared_open': (c_i32, [c_vp, ctypes.c_char_p, ctypes.POINTER(c_vp)]),
     'vr_shared_close': (c_i32, [c_vp, c_vp, c_i32]),
@@ -149,3 +153,12 @@ def stream_ptr():
 
 def ptr(t):
     return c_vp(t.data_ptr())
+
+
+def ptr_array(tensors):
+    """HOST array of the tensors' device pointers (None gives NULL), as vr_separate_many / vr_separate_waves take."""
+    return (c_vp * len(tensors))(*[None if t is None else t.data_ptr() for t in tensors])
+
+
+def i64_array(values):
+    return (c_i64 * len(values))(*[int(v) for v in values])
